@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU reference arm
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + the outputs as .npy
 
 Headline workload (BASELINE.json configs[1], "C1"): dense-mass Euclidean leapfrog on Neal's
 funnel, D = 128, 8192 chains per GPU, step size 0.01.  One bench "step" = one launch of
@@ -33,6 +34,10 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the tree (which may be read-only): no bytecode caches, here
+# or in the CPU baseline's spawned workers (they inherit the environment)
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 METRIC = "leapfrog steps/sec (aggregate over chains)"
 UNIT = "leapfrog steps/s"
@@ -82,7 +87,27 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-workloads", action="store_true",
                     help="headline workload only (skip C2 / C3 / C4 and strong scaling)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed launch returned on "
+                         "rank 0 (pos, mom, status, n_done of its chains) as DIR/<name>.npy in "
+                         "float64; the inputs are seeded, so runs with the same arguments can "
+                         "be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm")
+    return args
+
+
+def dump_outputs(out_dir, state):
+    """``state``'s arrays as float64 ``out_dir/<name>.npy`` (8192 chains, D = 128: 16 MB)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("pos", "mom", "status", "n_done"):
+        arr = getattr(state, name).detach().cpu().numpy().astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def measured_hbm_peak():
@@ -584,6 +609,10 @@ def run_cuda(args, rank, local_rank, world):
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
     total_ms = float(total_ms.item())
     assert int((out.status != 0).sum().item()) == 0 and bool(torch.isfinite(out.pos).all())
+    # every timed launch steps the same initial state, so `out` does not depend on how many
+    # launches ran before it
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
 
     # ---------------- end-to-end through the public API with HOST buffers
     pos_h = torch.as_tensor(prob.pos).pin_memory()

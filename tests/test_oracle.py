@@ -1,11 +1,12 @@
-"""CPU tests: the oracle port against the committed reference fixtures, the reference's own
-solver known answers, and (when /root/reference is present) the live reference."""
+"""CPU tests: the oracle port against the committed reference fixtures and the reference's own
+solver known answers."""
 
 import numpy as np
 import pytest
 
 from oracle import drivers as dr
 from oracle import mici_oracle as mo
+from oracle.make_golden import REFERENCE_5_STEP_CASES
 
 from golden_util import assert_matches_golden, case_names, load_case
 
@@ -82,15 +83,21 @@ def test_fixed_point_direct_handles_value_error():
         mo.solve_fixed_point_direct(func, np.array([1.0]))
 
 
-@pytest.mark.skipif(not dr.reference_available(), reason="reference tree not on this machine")
-@pytest.mark.parametrize("name", ["c1_funnel_dense_d24", "c2_softabs_banana_d8", "c3_torus_inner3"])
-def test_oracle_matches_live_reference(name):
+@pytest.mark.parametrize("name", REFERENCE_5_STEP_CASES)
+def test_oracle_matches_reference_5_steps(name):
+    """Five steps against the reference's own (tests/golden/reference_5_steps.npz), with tighter
+    tolerances than the step fixtures."""
+    import os
+
+    from oracle.make_golden import GOLDEN_DIR, input_checksum
+
     problem, dirs, overrides, _ = load_case(name)
-    r = dr.reference_run(problem, 5, dirs=dirs, **overrides)
+    r = np.load(os.path.join(GOLDEN_DIR, "reference_5_steps.npz"))
+    np.testing.assert_allclose(input_checksum(problem), r[f"{name}_input_checksum"], rtol=1e-13)
     o = dr.oracle_run(problem, 5, dirs=dirs, **overrides)
-    np.testing.assert_array_equal(o["status"], r["status"])
-    np.testing.assert_allclose(o["pos"], r["pos"], rtol=1e-13, atol=1e-15)
-    np.testing.assert_allclose(o["mom"], r["mom"], rtol=1e-13, atol=1e-15)
+    np.testing.assert_array_equal(o["status"], r[f"{name}_status"])
+    np.testing.assert_allclose(o["pos"], r[f"{name}_pos"], rtol=1e-13, atol=1e-15)
+    np.testing.assert_allclose(o["mom"], r[f"{name}_mom"], rtol=1e-13, atol=1e-15)
 
 
 @pytest.mark.parametrize("name", HMC_NAMES)
